@@ -22,6 +22,8 @@ un-vendored Ollama/llama.cpp behind HTTP, cannot be installed here: no node / ol
 Launch: python bench.py [--gpus N --steps K --warmup W]; N>1 via torchrun (one rank per GPU, no data-path collective: requests
 are independent, SURVEY.md section 8e) -- weak scaling.  `--workload config3 --gpus N` WITHOUT torchrun runs N engines in ONE
 process behind one scheduler (the north_star's in-process shape).
+`--dump-outputs DIR` writes what the last timed step returned (config2 / config4: token ids and logprobs; config5: the embeddings)
+as DIR/<name>.npy: the inputs are seeded, so two builds run with the same arguments can be compared output for output.
 """
 from __future__ import annotations
 
@@ -33,6 +35,7 @@ import os
 import statistics
 import subprocess
 import sys
+import tempfile
 import threading
 import time
 
@@ -40,6 +43,7 @@ import numpy as np
 
 ROOT = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, ROOT)
+sys.dont_write_bytecode = True          # the tree may be read-only: nothing is written beside the sources
 
 N_PROMPT, N_GEN = 512, 128
 MODEL_DIR = "/dev/shm" if os.path.isdir("/dev/shm") and os.access("/dev/shm", os.W_OK) else "/tmp"
@@ -111,6 +115,7 @@ class ClockSampler:
         if self.proc is None:
             return {"sm_mhz": None, "sm_max_mhz": None, "reasons": ["nvidia-smi unavailable"]}
         self.proc.terminate()
+        self.proc.wait()
         sm, mx, reasons = [], None, set()
         names = ["hw_slowdown", "hw_thermal_slowdown", "sw_thermal_slowdown", "sw_power_cap"]
         for r in self.rows:
@@ -146,19 +151,20 @@ def physical_cores() -> int:
 
 
 class CpuRestatement:
-    """oracle/c/llama_cpu.c on this box's host cores.  Prefers a -march=native build made here (oracle/_ref is git-ignored and
-    travels to the GPU box); falls back to the portable prebuilt library."""
+    """oracle/c/llama_cpu.c on this machine's host cores.  Prefers a -march=native build made at run time in a temporary
+    directory; falls back to the portable library build() made (oracle/_ref/liboracle_cpu.so)."""
 
     def __init__(self, path: str, n_ctx: int):
         src = os.path.join(ROOT, "oracle", "c", "llama_cpu.c")
         so = os.path.join(ROOT, "oracle", "_ref", "liboracle_cpu.so")
-        native = os.path.join(ROOT, "oracle", "_ref", f"liboracle_cpu_native_{os.getuid()}.so")
         lib = None
         try:
             cc = "/usr/bin/gcc" if os.path.exists("/usr/bin/gcc") else "gcc"
-            subprocess.check_call([cc, "-O3", "-march=native", "-fopenmp", "-fPIC", "-shared", "-o", native, src, "-lm"],
-                                  stdout=subprocess.DEVNULL, stderr=subprocess.DEVNULL, timeout=180)
-            lib = C.CDLL(native)
+            with tempfile.TemporaryDirectory(prefix="gridllm_bench_") as d:
+                native = os.path.join(d, "liboracle_cpu_native.so")
+                subprocess.check_call([cc, "-O3", "-march=native", "-fopenmp", "-fPIC", "-shared", "-o", native, src, "-lm"],
+                                      stdout=subprocess.DEVNULL, stderr=subprocess.DEVNULL, timeout=180)
+                lib = C.CDLL(native)            # stays mapped after the directory is removed
             so = native
         except Exception:
             lib = None
@@ -260,8 +266,13 @@ def main():
     ap.add_argument("--batch", type=int, default=32, help="config3: concurrent requests per GPU")
     ap.add_argument("--docs", type=int, default=1250, help="config5: documents per GPU per step (10 000 / 8 workers)")
     ap.add_argument("--batch-weights", type=int, default=0, help="config3: 0 auto, 1 resident 16-bit weights, 2 quantised weights")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write what the last step returned to its caller as DIR/<name>.npy (rank 0)")
     args = ap.parse_args()
     wl = args.workload
+    if args.dump_outputs and (args.impl != "native" or wl == "config3"):
+        # config3's callers receive streamed text, which the vocabulary-less synthetic model leaves empty
+        ap.error("--dump-outputs: native arm, workloads config2 / config4 / config5")
     # a stall must leave evidence: every thread's stack goes to stderr if the run makes no visible progress for a while
     import faulthandler
     faulthandler.enable()
@@ -353,12 +364,15 @@ def main():
         """barrier + synchronize, run, synchronize + barrier; clocks sampled on rank 0 during the region"""
         if rank == 0:
             sampler.start()
-        barrier()
-        torch.cuda.synchronize()
-        r = fn()
-        torch.cuda.synchronize()
-        barrier()
-        return r, (sampler.stop() if rank == 0 else None)
+        try:
+            barrier()
+            torch.cuda.synchronize()
+            r = fn()
+            torch.cuda.synchronize()
+            barrier()
+        finally:                                     # the polling nvidia-smi must not outlive a region that raised
+            clocks = sampler.stop() if rank == 0 else None
+        return r, clocks
 
     extra = {}
     if wl == "config2":
@@ -369,6 +383,8 @@ def main():
         out = run_config4(args, N, path, rank, local_rank, world, dist, timed, peaks, extra)
     else:
         out = run_config5(args, N, path, rank, local_rank, world, dist, timed, peaks, extra)
+    if rank == 0 and args.dump_outputs:
+        write_outputs(args.dump_outputs, out["outputs"])
     if rank == 0:
         line = {"metric": metric, "value": out["value"], "unit": unit, "n_gpus": out.get("n_gpus", world), "steps": args.steps, "warmup": args.warmup,
                 "ms_per_step": out["ms_per_step"], "higher_is_better": True, "scaling": "weak", "vs_baseline": None, "dtype": out["dtype"],
@@ -397,16 +413,33 @@ def prompt_for(i: int, n: int = N_PROMPT, vocab: int = 128000) -> np.ndarray:
     return np.random.Generator(np.random.PCG64(1000 + i)).integers(0, vocab, size=n).astype(np.int32)
 
 
+DUMP_BYTES = 60 << 20                   # array data: with the .npy headers the files stay below 64 MB (10^6 or 2^20 bytes)
+
+
+def write_outputs(out_dir: str, outputs: dict) -> None:
+    """--dump-outputs: one out_dir/<name>.npy per array, token ids as float64 (exact), everything else as float32.  Inputs are
+    seeded, so two builds run with the same arguments can be compared file by file.  Above DUMP_BYTES in all, each array keeps
+    a fixed, seeded sample of its rows, whose indices are written beside it as <name>_rows.npy."""
+    arrays = {k: np.asarray(v, np.float64 if np.issubdtype(np.asarray(v).dtype, np.integer) else np.float32) for k, v in outputs.items()}
+    total = sum(a.nbytes for a in arrays.values())
+    if total > DUMP_BYTES:
+        for k, a in list(arrays.items()):
+            keep = int(DUMP_BYTES * a.nbytes / total) // (a.nbytes // len(a) + 8)
+            rows = np.sort(np.random.Generator(np.random.PCG64(0)).choice(len(a), keep, replace=False))
+            arrays[k], arrays[f"{k}_rows"] = a[rows], rows.astype(np.float64)
+    os.makedirs(out_dir, exist_ok=True)
+    for k, a in arrays.items():
+        np.save(os.path.join(out_dir, f"{k}.npy"), a)
+    log(f"[bench] outputs of the last timed step: {', '.join(f'{k} {a.shape}' for k, a in arrays.items())} -> {out_dir}")
+
+
 # ---------------------------------------------------------------------------------------------------------------------
 def preflight_8b_parity(eng, path: str) -> dict:
     """The benchmarked model itself, GPU vs the C restatement in EXACT mode (dequantised fp32 weights x fp32 activations): 4 prompt
     tokens + 4 greedy tokens through the decode kernels at the full Llama-3-8B shape (32 layers, 128 256-entry vocabulary, K = 14336
     in 4 K-segments, GQA 4:1).  Tolerances of tests/test_gpu_decode.py: logits within 1e-2 * max|logit| of exact arithmetic, logprob
     within 2e-2, ids equal wherever the oracle's top-1/top-2 margin exceeds 5e-2.  Raises on a mismatch: a fast wrong kernel is not a result."""
-    so = os.path.join(ROOT, "oracle", "_ref", f"liboracle_cpu_native_{os.getuid()}.so")
-    if not os.path.exists(so):
-        so = os.path.join(ROOT, "oracle", "_ref", "liboracle_cpu.so")
-    lib = C.CDLL(so)
+    lib = C.CDLL(os.path.join(ROOT, "oracle", "_ref", "liboracle_cpu.so"))
     lib.oc_load.restype = C.c_void_p
     lib.oc_load.argtypes = [C.c_char_p, C.c_int]
     lib.oc_step.argtypes = [C.c_void_p, C.c_int, C.c_int, C.c_void_p, C.c_void_p]
@@ -496,7 +529,8 @@ def run_config2(args, N, path, rank, local_rank, world, dist, timed, peaks, extr
             "clocks": clocks,
             "extra": {"breakdown": {"prefill_ms_per_request": prefill_ns / args.steps * 1e-6, "decode_ms_per_request": (dev_ns - prefill_ns) / args.steps * 1e-6,
                                     "decode_tok_s_per_gpu": N_GEN / ((dev_ns - prefill_ns) / args.steps * 1e-9)},
-                      "parity_preflight": pre}}
+                      "parity_preflight": pre},
+            "outputs": {"ids": last.ids, "logprobs": last.logprobs}}
 
 
 # ---------------------------------------------------------------------------------------------------------------------
@@ -633,6 +667,7 @@ def run_config4(args, N, path, rank, local_rank, world, dist, timed, peaks, extr
     def region():
         dev_ns = wall = launches = 0
         for i in range(args.steps):
+            gens = []
             for s in range(S):
                 p = prompt_for(2000 + multirank.request_seeds(rank, i, 1)[0] * S + s, T)
                 t0 = time.perf_counter()
@@ -640,8 +675,9 @@ def run_config4(args, N, path, rank, local_rank, world, dist, timed, peaks, extr
                 wall += time.perf_counter() - t0
                 dev_ns += g.stats.prompt_eval_duration_ns
                 launches += g.stats.kernel_launches
-        return dev_ns, wall, launches
-    (dev_ns, wall_s, launches), clocks = timed(region)
+                gens.append(g)
+        return dev_ns, wall, launches, gens
+    (dev_ns, wall_s, launches, gens), clocks = timed(region)
     tokens = float(args.steps * S * T)
     agg = multirank.aggregate_throughput(tokens, dev_ns * 1e-9, wall_s, dist)
     qd, kvd = info.n_head * info.head_dim, info.n_head_kv * info.head_dim
@@ -657,7 +693,8 @@ def run_config4(args, N, path, rank, local_rank, world, dist, timed, peaks, extr
             "roofline": {"bound": "tensor", "kernel": "gemm_tc5_kernel (the prefill's linear layers: > 90 % of the step's flops); whole prefill timed",
                          "achieved": achieved, "peak": peaks["tf"], "unit": "TFLOP/s", "frac": achieved / peaks["tf"], "peak_source": peaks["src"],
                          "algorithmic_flops_per_step": flops_seq * S, "traffic": None},
-            "clocks": clocks, "extra": {}}
+            "clocks": clocks, "extra": {},
+            "outputs": {"ids": np.concatenate([g.ids for g in gens]), "logprobs": np.concatenate([g.logprobs for g in gens])}}
 
 
 def run_config5(args, N, path, rank, local_rank, world, dist, timed, peaks, extra):
@@ -674,7 +711,7 @@ def run_config5(args, N, path, rank, local_rank, world, dist, timed, peaks, extr
     def region():
         dev_ns = wall = launches = n = 0
         for i in range(args.steps):
-            k = 0
+            k, embs = 0, []
             while k < args.docs:
                 d = docs(i, k, min(pack, args.docs - k))
                 t0 = time.perf_counter()
@@ -684,9 +721,10 @@ def run_config5(args, N, path, rank, local_rank, world, dist, timed, peaks, extr
                 launches += st.kernel_launches
                 n += len(d)
                 k += len(d)
+                embs.append(emb)
         assert np.isfinite(emb).all()
-        return dev_ns, wall, launches, n
-    (dev_ns, wall_s, launches, n), clocks = timed(region)
+        return dev_ns, wall, launches, n, embs
+    (dev_ns, wall_s, launches, n, embs), clocks = timed(region)
     agg = multirank.aggregate_throughput(float(n), dev_ns * 1e-9, wall_s, dist)
     qd, kvd = info.n_head * info.head_dim, info.n_head_kv * info.head_dim
     lin_params = info.n_layer * ((qd + 2 * kvd) * info.n_embd + info.n_embd * qd + 3 * info.n_ff * info.n_embd)
@@ -701,7 +739,7 @@ def run_config5(args, N, path, rank, local_rank, world, dist, timed, peaks, extr
             "roofline": {"bound": "tensor", "kernel": "gemm_tc5_kernel (packed prompt pass); whole gl_embed device time", "achieved": achieved,
                          "peak": peaks["tf"], "unit": "TFLOP/s", "frac": achieved / peaks["tf"], "peak_source": peaks["src"],
                          "algorithmic_flops_per_doc": flops_doc, "traffic": None},
-            "clocks": clocks, "extra": {"docs_per_call": pack}}
+            "clocks": clocks, "extra": {"docs_per_call": pack}, "outputs": {"embeddings": np.concatenate(embs)}}
 
 
 if __name__ == "__main__":

@@ -77,17 +77,15 @@ def tiny_f16_gguf(tmp_models):
 
 
 @pytest.fixture(scope="session")
-def hostcheck_lib():
-    """CPU build of the GEMV lane program (tests/hostcheck) -- test infrastructure only."""
+def hostcheck_lib(tmp_path_factory):
+    """CPU build of the GEMV lane program (tests/hostcheck) -- test infrastructure only.  Built afresh every session, outside
+    the tree, so it always matches the product headers it includes."""
     import ctypes
     src = os.path.join(ROOT, "tests", "hostcheck", "hostcheck.cpp")
-    out = os.path.join(ROOT, "tests", "hostcheck", "libhostcheck.so")
-    deps = [src, os.path.join(ROOT, "gridllm_b200", "csrc", "rowdot.h"), os.path.join(ROOT, "gridllm_b200", "csrc", "gguf_file.cpp"),
-            os.path.join(ROOT, "gridllm_b200", "csrc", "tokenizer.cpp"), os.path.join(ROOT, "gridllm_b200", "csrc", "unicode_ranges.h")]
-    if not os.path.exists(out) or any(os.path.getmtime(d) > os.path.getmtime(out) for d in deps):
-        subprocess.check_call(["g++", "-O2", "-std=c++17", "-shared", "-fPIC", "-o", out, src,
-                               os.path.join(ROOT, "gridllm_b200", "csrc", "gguf_file.cpp"),
-                               os.path.join(ROOT, "gridllm_b200", "csrc", "tokenizer.cpp")])
+    out = str(tmp_path_factory.mktemp("hostcheck") / "libhostcheck.so")
+    subprocess.check_call(["g++", "-O2", "-std=c++17", "-shared", "-fPIC", "-o", out, src,
+                           os.path.join(ROOT, "gridllm_b200", "csrc", "gguf_file.cpp"),
+                           os.path.join(ROOT, "gridllm_b200", "csrc", "tokenizer.cpp")])
     return ctypes.CDLL(out)
 
 
